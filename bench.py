@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU path, same metric
+    python bench.py ... --dump-outputs DIR                    # also save the last timed step's results as .npy
 
 Workload (config.workload): BASELINE.json configs[2], the one the metric is quoted on -- a 10M-entry
 GFKB of synthetic failures.jsonl-shaped ``signature_text`` rows, a 100k-query batch, the reference's
@@ -14,6 +15,11 @@ fixed): per-shard scan -> one all-gather of partial top-k -> merge.
 scan + merge [+ all-gather + merge]); ``e2e``: queries/s through the public API from host text
 buffers (host featurisation, host->device copies, kernels, device->host read of the result).
 Only the ``cpu_baseline`` / ``--impl reference`` legs execute anything under oracle/.
+
+``--dump-outputs DIR`` writes what the last timed step returned: ``scores.npy`` (float32 [Q, k]) and ``rows.npy``
+(global row ids as float64 [Q, k], -1 = no row).  The inputs are generated from fixed seeds, so two builds run with
+the same arguments can be compared output for output.  Past 64 MB a fixed, seeded sample of the queries is written,
+and ``query_index.npy`` (float64) lists the sampled queries.
 """
 from __future__ import annotations
 
@@ -28,21 +34,34 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True   # the benchmark leaves the tree it runs from untouched
 
 METRIC = "fingerprint-match queries/sec over 10M-entry GFKB"
 UNIT = "queries/s"
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def _count(minimum):
+    def parse(s):
+        v = int(s)
+        if v < minimum:
+            raise argparse.ArgumentTypeError(f"must be >= {minimum}, got {v}")
+        return v
+    return parse
 
 
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=_count(1), default=3, help="timed steps (resident path; also the end-to-end calls unless --e2e-steps is given)")
+    ap.add_argument("--warmup", type=_count(0), default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--rows", type=int, default=10_000_000)
     ap.add_argument("--queries", type=int, default=100_000)
     ap.add_argument("--k", type=int, default=16)
-    ap.add_argument("--e2e-steps", type=int, default=3)
+    ap.add_argument("--e2e-steps", type=_count(1), default=None, help="timed end-to-end calls from host text (default: --steps)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's top-k (scores.npy float32, rows.npy float64) to DIR")
     ap.add_argument("--cpu-sample-rows", type=int, default=50_000)
     ap.add_argument("--cpu-sample-queries", type=int, default=4)
     ap.add_argument("--no-cpu-baseline", action="store_true")
@@ -50,7 +69,30 @@ def parse_args():
     ap.add_argument("--shard", default="rows", choices=["rows", "queries", "rows-text"],
                     help="rows: corpus rows sharded over the GPUs by row index (BASELINE configs[2]); rows-text: sharded by ranges of "
                          "the global text order (tighter chunks per shard); queries: index replicated, queries split")
-    return ap.parse_args()
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs saves the top-k of the CUDA path; the reference arm computes no top-k")
+    if a.e2e_steps is None:
+        a.e2e_steps = a.steps
+    return a
+
+
+def dump_outputs(out_dir, scores, rows):
+    """scores float32 [Q, k], rows int64 [Q, k] -> DIR/scores.npy, DIR/rows.npy (float64: row ids < 2^53 are exact).
+    Above DUMP_LIMIT_BYTES a seeded sample of the queries (in query order) is kept and listed in query_index.npy."""
+    import numpy as np
+
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    q, k = scores.shape
+    per_query = k * (4 + 8)
+    budget = DUMP_LIMIT_BYTES - 4096          # room for the .npy headers
+    if q * per_query > budget:
+        keep = np.sort(np.random.default_rng(0).choice(q, budget // (per_query + 8), replace=False))
+        scores, rows = scores[keep], rows[keep]
+        np.save(out / "query_index.npy", keep.astype(np.float64))
+    np.save(out / "scores.npy", np.ascontiguousarray(scores, dtype=np.float32))
+    np.save(out / "rows.npy", np.ascontiguousarray(rows, dtype=np.float64))
 
 
 def workload_config(a, world):
@@ -134,10 +176,16 @@ def _standalone_synth(seed, count, dup_of_seed=0, dup_rows=0):
     import numpy as np
 
     so = ROOT / "oracle" / "_build" / "libkvsynth.so"
-    if not so.exists():
-        subprocess.run(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-pthread", str(ROOT / "oracle" / "synth_shim.cpp"),
-                        "-o", str(so)], check=True)
-    lib = C.CDLL(str(so))
+    if so.exists():
+        lib = C.CDLL(str(so))
+    else:   # not built: compile into a temporary directory, never into the tree
+        import tempfile
+
+        with tempfile.TemporaryDirectory(prefix="kvsynth-") as tmp:
+            so = Path(tmp) / "libkvsynth.so"
+            subprocess.run(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-pthread", str(ROOT / "oracle" / "synth_shim.cpp"),
+                            "-o", str(so)], check=True)
+            lib = C.CDLL(str(so))
     lib.kv_synth_signatures.restype = C.c_int
     lib.kv_synth_signatures.argtypes = [C.c_uint64, C.c_int64, C.c_int64, C.c_uint64, C.c_int64, C.c_char_p, C.c_int64,
                                         C.POINTER(C.c_int64)]
@@ -348,6 +396,8 @@ def run_ours(a):
     n_check = min(64, a.queries)
     ok_pairs = bad = 0
     s_h, r_h = s.cpu().numpy(), r.cpu().numpy()
+    if a.dump_outputs and rank == 0:   # every rank holds the same merged result
+        dump_outputs(a.dump_outputs, s_h, r_h)
     row_map = shard.row_map.cpu().numpy() if getattr(shard, "row_map", None) is not None else None
     base = shard.index.row_base if hasattr(shard.index, "row_base") else 0
     for qi in np.linspace(0, a.queries - 1, n_check).astype(np.int64):
@@ -376,7 +426,7 @@ def run_ours(a):
     assert bad_total == 0, f"in-run parity check failed on {bad_total} item(s)"
 
     # ---- end to end from host text ----
-    e2e_steps = max(1, a.e2e_steps)
+    e2e_steps = a.e2e_steps
     for _ in range(2):  # warm-up (staging and read-back buffers of both parities get pinned here, not in the timed calls)
         shard.topk_packed(qbuf, qoff, a.k)
     barrier()
@@ -731,7 +781,7 @@ def run_ours(a):
             "warmup": a.warmup, "ms_per_step": step_ms, "higher_is_better": True, "scaling": "strong",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": cfg, "clocks": clocks,
             "e2e": {"value": a.queries / e2e_s, "unit": UNIT, "h2d_bytes_per_step": int(h2d), "d2h_bytes_per_step": int(d2h),
-                    "ms_per_step": e2e_s * 1e3, "rank0_split_ms": getattr(shard, "last_e2e_ms", None),
+                    "steps": e2e_steps, "ms_per_step": e2e_s * 1e3, "rank0_split_ms": getattr(shard, "last_e2e_ms", None),
                     "rank0_ms_per_call": e2e_calls},
             "gpu_launches": int(lay["kernel_launches"] + (1 if world > 1 else 0)) * a.steps,
             "roofline": roofline, "rank_stats": rank_stats, "parity_in_run": parity, "cpu_baseline": cpu, "secondary": secondary, "secondary_multi_gpu": secondary_multi,
